@@ -4,6 +4,7 @@ random-init weights of the reference architecture.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 8] [--precision strict|fast] [--impl ours|reference|torch_gpu]
     python bench.py --train [--gpus N] [--graph 1|0] ...                       # BASELINE configs[2] / configs[4]
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step returned to DIR/<name>.npy
 
 Inference (configs[1]; --batch 32 = configs[3]): a "step" = one pass of DLA-34 + IDA-up + DCNv2 + predictor + NMS / top-k / 3D
 decode over one batch. ONE JSON line (rank 0):
@@ -85,6 +86,16 @@ def cpu_threads():
     """torch-CPU convolutions stop scaling (and the gather-heavy DCN restatement regresses) beyond ~32 threads:
     measured 91 s/img with 128 threads vs 19 s/img with fewer on the round-1 box. Use at most 32."""
     return min(os.cpu_count() or 1, 32)
+
+
+def dump_outputs(out_dir, arrays):
+    """{name: array} -> out_dir/<name>.npy, float32 arrays as they are and everything else as float64. The inputs are
+    seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ CPU reference path
@@ -373,6 +384,9 @@ def bench_train(args, rank, world, local_rank, config):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:          # the captured step re-uses its loss buffers: read them before the next step
+        dump_outputs(args.dump_outputs, dict([("loss_" + k, v.float().cpu().numpy()) for k, v in loss_dict.items()] +
+                                             [("log_" + k, v) for k, v in log.resolve().items()]))
     barrier()
     # exposed gradient-exchange time: the NCCL all-reduce of the arena alone, same buckets (N > 1)
     ms_ar = 0.0
@@ -485,8 +499,9 @@ def bench_train(args, rank, world, local_rank, config):
 
 
 # ------------------------------------------------------------------------------------------------ inference bench
-def time_inference(model, targets, host_imgs, dev_imgs, steps, B, dev, barrier):
-    """-> (ms device-resident, ms end-to-end, d2h bytes) for `steps` forwards of `model` in its current precision"""
+def time_inference(model, targets, host_imgs, dev_imgs, steps, B, dev, barrier, keep_last=False):
+    """-> (ms device-resident, ms end-to-end, d2h bytes, last) for `steps` forwards of `model` in its current precision;
+    `last` is what `forward_async(...).result()` returned for the last device-resident step if `keep_last`, else None"""
     import torch
     n_in = len(dev_imgs)
     with torch.no_grad():
@@ -498,10 +513,11 @@ def time_inference(model, targets, host_imgs, dev_imgs, steps, B, dev, barrier):
     e0.record()
     with torch.no_grad():
         for i in range(steps):
-            model.forward_async(dev_imgs[i % n_in], targets)          # no host sync inside the device-resident loop
+            pending = model.forward_async(dev_imgs[i % n_in], targets)    # no host sync inside the device-resident loop
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
+    last = pending.result() if keep_last else None     # before the next forward re-uses the decode workspace
     barrier()
     # end to end: pinned host -> H2D (copy stream, one batch ahead) -> model -> D2H of the detections
     copy_stream = torch.cuda.Stream(device=dev)
@@ -544,7 +560,7 @@ def time_inference(model, targets, host_imgs, dev_imgs, steps, B, dev, barrier):
     torch.cuda.synchronize()
     ms_e2e = t0.elapsed_time(t1)
     barrier()
-    return ms, ms_e2e, B * 50 * 14 * 4 + 4 * B
+    return ms, ms_e2e, B * 50 * 14 * 4 + 4 * B, last
 
 
 def main():
@@ -562,7 +578,12 @@ def main():
     ap.add_argument("--sync-bn", type=int, default=1, help="--train, N > 1: SyncBatchNorm like the reference's yaml (1, default) or per-GPU statistics (0)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--dump-launches", default=None, help="write the per-launch timing table (json) to this path")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy: the detections "
+                         "and per-image counts, or with --train the loss terms and logged scalars")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the project's own path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -621,7 +642,11 @@ def main():
     with torch.no_grad():
         for i in range(max(3, args.warmup)):
             model(dev_imgs[i % n_in], targets)
-    ms, ms_e2e, d2h = time_inference(model, targets, host_imgs, dev_imgs, args.steps, B, dev, barrier)
+    ms, ms_e2e, d2h, last = time_inference(model, targets, host_imgs, dev_imgs, args.steps, B, dev, barrier,
+                                           keep_last=bool(args.dump_outputs) and rank == 0)
+    if last is not None:
+        rows, counts = last
+        dump_outputs(args.dump_outputs, {"detections": rows.numpy(), "detections_per_image": counts})
     launches_per_step = model.backbone.last_plan.n_launch + model.heads.predictor.last_plan.n_launch + 1 + 2
     if rank == 0:
         sampler.stop_flag = True
@@ -694,7 +719,7 @@ def main():
     # ---------------------------------------------------------------- the other precision (fewer steps: context number)
     model.set_precision(other)
     steps2 = max(5, args.steps // 2)
-    ms2, ms2_e2e, _ = time_inference(model, targets, host_imgs, dev_imgs, steps2, B, dev, barrier)
+    ms2, ms2_e2e, _, _ = time_inference(model, targets, host_imgs, dev_imgs, steps2, B, dev, barrier)
     ms2, ms2_e2e = parallel.max_over_ranks([ms2, ms2_e2e], device=dev)
     modes[other] = {"value": world * B * steps2 / (ms2 * 1e-3), "e2e": world * B * steps2 / (ms2_e2e * 1e-3),
                     "ms_per_step": ms2 / steps2, "steps": steps2}

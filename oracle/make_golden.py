@@ -39,6 +39,20 @@ def ref_targets(tg):
     return out
 
 
+def dcn_columns():
+    """The reference's modulated_deformable_im2col_cpu columns of the dcn_op.npz inputs -> dcn_cols.npz, so the sampling
+    step of oracle.dcn_columns stays pinned to the reference's C loops without the compiled library."""
+    lib = rs._load_ref_so()
+    with np.load(os.path.join(OUT, "dcn_op.npz")) as z:
+        x, off, mask = (np.ascontiguousarray(z[k]) for k in ("x", "offset", "mask"))
+    B, C, H, W = x.shape
+    cols = np.empty((B, C * 9, H * W), np.float32)
+    for b in range(B):
+        lib.modulated_deformable_im2col_cpu(x[b].ctypes.data, off[b].ctypes.data, mask[b].ctypes.data, 1, C, H, W, H, W,
+                                            3, 3, 1, 1, 1, 1, 1, 1, 1, cols[b].ctypes.data)
+    np.savez_compressed(os.path.join(OUT, "dcn_cols.npz"), cols=cols)
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
@@ -55,6 +69,7 @@ def main():
     y = _ext.dcn_v2_forward(x, w, bias, off, mask, 3, 3, 1, 1, 1, 1, 1, 1, 1)
     np.savez_compressed(os.path.join(OUT, "dcn_op.npz"), x=x.numpy(), offset=off.numpy(), mask=mask.numpy(), weight=w.numpy(),
                         bias=bias.numpy(), y=y.numpy())
+    dcn_columns()
 
     # ---------------------------------------------------------------- 2. whole detector, eval, 1x3x128x256
     Hh, Ww, Bb = 128, 256, 1
