@@ -25,13 +25,6 @@ const char* mf_last_error(void);
 int mf_version(void);
 /* 0 = tcgen05 tensor-core implicit GEMM (default, the product), 1 = CUDA-core cross-check kernels (diagnostics). */
 int mf_set_conv_impl(int impl);
-/* performance tunables (experiments; results never depend on them): id 0/1 = extra dynamic shared memory (bytes) for
- * DCN / conv CTAs (fewer resident CTAs, larger L1); id 2 = unused (was the first-generation non-persistent GEMM kernel, removed);
- * id 3 = 1 disables the TMA-store epilogue; id 4 = 1 disables the im2col-TMA A operand (cp.async gather instead); id 5 = 1 also uses
- * im2col TMA for Cin 8/16/32 (request-bound, slower); id 6 = 1 enables the A-stationary schedule of wide-N GEMMs (measured slower: too
- * few B bytes in flight); id 7 = 2 runs the DCN gather with 8 producer warps instead of 16; id 8 = 1 launches with programmatic dependent launch (no measured gain under graph replay);
- * id 9 = 1 runs the fused head as 2-CTA clusters that TMA-multicast the 3x3 weight boxes (halves their L2->SM traffic). */
-int mf_set_tunable(int id, int value);
 /* N tile (16/32/64/128) the conv kernels use for `cout`; packed weights / scale / shift are padded to a multiple. */
 int mf_conv_block_n(int cout);
 

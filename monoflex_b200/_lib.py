@@ -15,7 +15,6 @@ SIGNATURES = {
     "mf_version": [],
     "mf_set_conv_impl": [_I],
     "mf_conv_block_n": [_I],
-    "mf_set_tunable": [_I, _I],
     "mf_pack_conv_weight": [_P, _I, _I, _I, _I, _I, _I, _I, _P, _P],
     "mf_pack_conv_weight_dgrad": [_P, _I, _I, _I, _I, _I, _I, _I, _P, _P],
     "mf_pack_conv_weights_batched": [_P, _I, _P],
@@ -106,9 +105,6 @@ def load():
             fn.argtypes = args
             fn.restype = _SZ if name.endswith("_workspace") else _I
         _lib = lib
-        for i, name in enumerate(("MF_DCN_EXTRA_SMEM", "MF_CONV_EXTRA_SMEM", "MF_UNUSED_2", "MF_NO_TMA_STORE", "MF_NO_TMA_IM2COL", "MF_TMA_SMALL_C", "MF_A_STATIONARY", "MF_DCN_WARPS_MODE", "MF_PDL", "MF_HEAD_CLUSTER", "MF_WGRAD_NO_NARROW", "MF_SPLIT_KCONCAT", "MF_HEAD2_BN256", "MF_PATCH")):     # experiments only
-            if os.environ.get(name):
-                lib.mf_set_tunable(i, int(os.environ[name]))
         if os.environ.get("MF_CONV_IMPL"):            # diagnostics only: 1 = CUDA-core cross-check kernels
             lib.mf_set_conv_impl(int(os.environ["MF_CONV_IMPL"]))
     return _lib

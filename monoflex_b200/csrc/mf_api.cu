@@ -98,8 +98,6 @@ int launch_pack_conv_weight_batched(const long long* descs, int n, cudaStream_t 
 
 // boundary B (exact-fp32 `_ext.dcn_v2_forward/backward` on NCHW tensors): kernels and launchers live in mf_dcn_f32.cu
 
-int g_tunable[16] = {0};   // experiment switches, see mf_set_tunable in include/monoflex_b200.h
-
 int igemm_block_n(int cout) {
   if (cout <= 16) return 16;
   if (cout <= 32) return 32;
@@ -127,11 +125,6 @@ int mf_set_conv_impl(int impl) {
   return 0;
 }
 int mf_conv_block_n(int cout) { return igemm_block_n(cout); }
-int mf_set_tunable(int id, int value) {
-  if (id < 0 || id >= 16) { set_error("mf_set_tunable: id out of range"); return -1; }
-  g_tunable[id] = value;
-  return 0;
-}
 
 int mf_pack_conv_weight(const float* w_oihw, int Cout, int Cin, int kh, int kw, int cin_pad, int n_pad, int k_pad,
                         void* out_f16, void* stream) {

@@ -40,7 +40,6 @@ __global__ void __launch_bounds__(256) bn_partial_kernel(const __half* __restric
                                                          const float* __restrict__ mean, const float* __restrict__ rstd,
                                                          long long M, int C, int act, long long rows_per_cta,
                                                          float* __restrict__ part) {
-  pdl_wait();
   extern __shared__ float sm[];                            // [RL][2][C]
   const int CV = C / 8, RL = blockDim.x / CV;
   const int cv = threadIdx.x % CV, r = threadIdx.x / CV;
@@ -141,7 +140,6 @@ __global__ void bn_finalize_kernel(const float* __restrict__ part, int ncta, int
 __global__ void __launch_bounds__(256) bn_apply_kernel(const __half* __restrict__ x, int x_ld, const float* __restrict__ scale,
                                                        const float* __restrict__ shift, const __half* __restrict__ res,
                                                        int res_ld, int act, __half* __restrict__ y, int y_ld, long long M, int C) {
-  pdl_wait();
   const int CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= M * CV) return;
@@ -187,7 +185,6 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const __half* __restr
                                                            const float* __restrict__ sum_gx, int act, __half* __restrict__ dx,
                                                            int dx_ld, __half* __restrict__ dres, int dres_ld, long long M, int C,
                                                            double count) {
-  pdl_wait();
   const int CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= M * CV) return;

@@ -36,7 +36,6 @@ MF_DEVINL uint4 bm_pack8(const float (&f)[8]) {
 __global__ void __launch_bounds__(256) maxpool2_bwd_kernel(const __half* __restrict__ x, const __half* __restrict__ dy,
                                                            __half* __restrict__ dx, int B, int H, int W, int C, int x_ld,
                                                            int dy_ld, int dx_ld) {
-  pdl_wait();
   const int Ho = H / 2, Wo = W / 2, CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Ho * Wo * CV) return;
@@ -79,7 +78,6 @@ int launch_maxpool2_bwd(const __half* x, const __half* dy, __half* dx, int B, in
 __global__ void __launch_bounds__(256) upsample_bwd_dx_kernel(const __half* __restrict__ dy, const float* __restrict__ w,
                                                               __half* __restrict__ dx, int B, int Hi, int Wi, int C, int f,
                                                               int dy_ld, int dx_ld) {
-  pdl_wait();
   const int CV = C / 8, k = 2 * f, pad = f / 2, Ho = Hi * f, Wo = Wi * f;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Hi * Wi * CV) return;
@@ -117,7 +115,6 @@ static constexpr int UPW_TAPS = 8;
 __global__ void __launch_bounds__(256) upsample_bwd_dw_kernel(const __half* __restrict__ x, const __half* __restrict__ dy,
                                                               float* __restrict__ part, int B, int Hi, int Wi, int C, int f,
                                                               int x_ld, int dy_ld, long long pix_per_slab) {
-  pdl_wait();
   const int CV = C / 8, k = 2 * f, pad = f / 2, Ho = Hi * f, Wo = Wi * f, taps = k * k;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int cv = blockIdx.x * 8 + warp;
@@ -225,7 +222,6 @@ int launch_upsample_bwd(const __half* x, const float* w, const __half* dy, __hal
 // ---------------------------------------------------------------- sigmoid_hm backward (fp32, any layout)
 __global__ void sigmoid_clamp_bwd_kernel(const float* __restrict__ y, const float* __restrict__ dy, float* __restrict__ dx,
                                          long long n) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float s = y[i];
@@ -239,7 +235,6 @@ int launch_sigmoid_clamp_bwd(const float* y, const float* dy, float* dx, long lo
 // ---------------------------------------------------------------- column sum of an [M, C] fp16 matrix
 __global__ void __launch_bounds__(256) column_sum_partial_kernel(const __half* __restrict__ x, int x_ld, long long M, int C,
                                                                  long long rows_per_cta, float* __restrict__ part) {
-  pdl_wait();
   const int CV = C / 8;
   const int cv = threadIdx.x % CV, r = threadIdx.x / CV, RL = blockDim.x / CV;
   extern __shared__ float sm[];                                            // [RL][C]
@@ -293,7 +288,6 @@ int launch_column_sum(const __half* x, int x_ld, long long M, int C, float* out,
 __global__ void edge_gather_bwd_kernel(const __half* __restrict__ d_ea, const __half* __restrict__ d_eb, int ch_a, int ch_b,
                                        const long long* __restrict__ edge_idx, __half* __restrict__ d_feat, int feat_ld, int B,
                                        int H, int W, int K, int out_w, int out_h) {
-  pdl_wait();
   const int CV = 32;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * (K + 2) * CV * 2) return;
@@ -347,7 +341,6 @@ __global__ void __launch_bounds__(256) edge_head_add_bwd_kernel(const __half* __
   // 8 warps per CTA, each walking EDGE_PER_WARP consecutive (b, e) positions: the weight / bias gradients are summed in
   // registers, then across the CTA's warps in shared memory, and only one atomic per (o, c) per CTA reaches `dw` (the
   // first version issued one per position: ~6.6 k warps hammering the same 768 addresses, 0.9 ms per launch).
-  pdl_wait();
   constexpr int EDGE_PER_WARP = 8;
   __shared__ float red[8][NO][256 + 1];
   __shared__ float redb[8][NO];
@@ -422,7 +415,6 @@ int launch_edge_head_add_bwd(const __half* t, const float* w, int n_out, const l
 // ---------------------------------------------------------------- dst[r, 0:C] += src[r, 0:C] (gradient accumulation)
 __global__ void __launch_bounds__(256) add_rows_kernel(__half* __restrict__ dst, int dst_ld, const __half* __restrict__ src,
                                                        int src_ld, long long M, int C) {
-  pdl_wait();
   const int CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= M * CV) return;
@@ -448,7 +440,6 @@ __global__ void __launch_bounds__(256) interleave2x2_kernel(const __half* __rest
                                                             const __half* __restrict__ p10, const __half* __restrict__ p11,
                                                             int part_ld, __half* __restrict__ out, int out_ld, int B, int Hh,
                                                             int Wh, int C) {
-  pdl_wait();
   const int CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Hh * Wh * CV) return;

@@ -13,9 +13,8 @@ namespace mf {
 // ------------------------------------------------------------------------------------------------ error state
 void set_error(const char* fmt, ...);
 int check_cuda(cudaError_t e, const char* what);
-extern int g_tunable[16];
 
-// <<<>>> replacement that can add the programmatic-stream-serialization attribute (tunable 8 == 1 turns it on)
+// <<<>>> replacement through cudaLaunchKernelEx
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg;
@@ -23,23 +22,12 @@ inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = g_tunable[8] == 1 ? 1 : 0;       // measured: no gain under CUDA-graph replay (A/B 1588 vs 1595 img/s) -> opt-in
+  cfg.attrs = nullptr;
+  cfg.numAttrs = 0;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
 MF_DEVINL uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-// ------------------------------------------------------------------------------------------------ programmatic dependent launch
-// With tunable 8 every kernel of the plan is launched with cudaLaunchAttributeProgrammaticStreamSerialization: it may start
-// while its predecessor is still draining (without the attribute the two instructions below are no-ops). `pdl_launch_dependents()` (first statement) lets the successor's CTAs be scheduled as
-// soon as SM resources free up; `pdl_wait()` blocks until the predecessor grid has completed and its writes are visible,
-// and must precede the first access to any buffer another kernel produces or still reads.
-MF_DEVINL void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-MF_DEVINL void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 // ------------------------------------------------------------------------------------------------ mbarrier
 MF_DEVINL void mbar_init(uint64_t* bar, uint32_t count) {
@@ -158,32 +146,6 @@ MF_DEVINL bool elect_one() {
       "}\n"
       : "=r"(pred));
   return pred != 0;
-}
-
-// ------------------------------------------------------------------------------------------------ thread-block clusters
-MF_DEVINL uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-MF_DEVINL void cluster_sync_all() {   // every thread of every CTA of the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// tiled 2D load whose box lands at the same smem offset in every CTA of `cta_mask`, completing tx bytes on each one's mbarrier
-MF_DEVINL void tma_load_2d_mc(uint32_t dst_smem, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], "
-      "[%2], %5;" ::"r"(dst_smem),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-      : "memory");
-}
-// tcgen05.commit arriving on the mbarrier at this offset in every CTA of `cta_mask`
-MF_DEVINL void umma_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(cta_mask)
-               : "memory");
 }
 
 // ------------------------------------------------------------------------------------------------ named barriers, TMA store, im2col-mode TMA load

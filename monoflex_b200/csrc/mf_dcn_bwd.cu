@@ -61,7 +61,6 @@ MF_DEVINL void dcn_unpack8(const uint4& v, float (&f)[8]) {
 // one thread per (pixel, tap, 8-channel chunk)
 __global__ void __launch_bounds__(256) dcn_sample_cols_kernel(const __half* __restrict__ x, int x_ld, const float* __restrict__ om,
                                                               int om_ld, __half* __restrict__ cols, int B, int H, int W, int C) {
-  pdl_wait();
   const int CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * H * W * 9 * CV) return;
@@ -98,7 +97,6 @@ __global__ void __launch_bounds__(256) dcn_sample_cols_kernel(const __half* __re
 __global__ void __launch_bounds__(256) dcn_col2im_kernel(const __half* __restrict__ x, int x_ld, const float* __restrict__ om,
                                                          int om_ld, const __half* __restrict__ gcol, __half* __restrict__ dx,
                                                          int dx_ld, float* __restrict__ dom, int B, int H, int W, int C, int L) {
-  pdl_wait();
   const int CV = C / 8;
   const long long gid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   const long long item = gid / L;

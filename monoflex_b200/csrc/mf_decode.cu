@@ -22,7 +22,6 @@ static constexpr int S1_CAND = 2048;                   // candidate-list capacit
 __global__ void __launch_bounds__(S1_THREADS)
 nms_topk_stage1_kernel(const float* __restrict__ hm_all, int H, int W, int K, int apply_sigmoid, int slabs,
                        float* __restrict__ out_score, int* __restrict__ out_idx) {
-  pdl_wait();
   // blockIdx.x = plane * slabs + slab; a slab is a contiguous pixel range [lo, hi) of one (image, class) plane. The union
   // of the per-slab top-K sets contains the plane's top-K, so splitting only adds parallelism (148 SMs instead of B*C).
   const int HW = H * W;
@@ -220,7 +219,6 @@ nms_topk_stage1_kernel(const float* __restrict__ hm_all, int H, int W, int K, in
 
 // stand-alone nms_hm (model/layers/utils.py:45-58): out = heat * (maxpool3x3(heat) == heat)
 __global__ void nms_hm_kernel(const float* __restrict__ hm, float* __restrict__ out, int H, int W, long long n) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int HW = H * W;
@@ -270,7 +268,6 @@ static constexpr int S2_THREADS = 1024;
 static constexpr int S2_KEYS = 2048;
 
 __global__ void __launch_bounds__(S2_THREADS) topk_decode_stage2_kernel(const DecodeParams p) {
-  pdl_wait();
   const int b = blockIdx.x;
   const int SK = p.S * p.K, CSK = p.C * SK;     // candidates per class / per image (<= 2048)
   __shared__ unsigned long long sel[S2_KEYS];

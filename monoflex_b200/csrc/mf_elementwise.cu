@@ -23,7 +23,6 @@ MF_DEVINL uint4 pack8(const float (&f)[8]) {
 
 // ---------------------------------------------------------------- image: NCHW fp32 [B,3,H,W] -> NHWC fp16 [B,H,W,8]
 __global__ void pack_image_kernel(const float* __restrict__ x, __half* __restrict__ y, int B, int C, long long HW) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B * HW) return;
   const long long b = i / HW, pix = i - b * HW;
@@ -41,7 +40,6 @@ int launch_pack_image(const float* x, __half* y, int B, int C, int H, int W, cud
 
 // ---------------------------------------------------------------- generic NCHW fp32 <-> NHWC fp16 (tile transpose)
 __global__ void nchw_to_nhwc_kernel(const float* __restrict__ x, __half* __restrict__ y, int C, int HW, int y_ld) {
-  pdl_wait();
   __shared__ float tile[32][33];
   const int b = blockIdx.z, p0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -60,7 +58,6 @@ int launch_nchw_to_nhwc(const float* x, __half* y, int B, int C, int HW, int y_l
   return check_cuda(cudaGetLastError(), "nchw_to_nhwc");
 }
 __global__ void nhwc_to_nchw_kernel(const __half* __restrict__ x, float* __restrict__ y, int C, int HW, int x_ld) {
-  pdl_wait();
   __shared__ float tile[32][33];
   const int b = blockIdx.z, p0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {
@@ -82,7 +79,6 @@ int launch_nhwc_to_nchw(const __half* x, float* y, int B, int C, int HW, int x_l
 // offset [B,18,H,W] + mask [B,9,H,W] (fp32 NCHW, reference _ext layout) -> [B*H*W, 32] fp32 rows
 __global__ void pack_offmask_kernel(const float* __restrict__ off, const float* __restrict__ mask, float* __restrict__ y,
                                     int B, int HW) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * HW * 32) return;
   const int ch = static_cast<int>(i & 31);
@@ -102,7 +98,6 @@ int launch_pack_offmask(const float* off, const float* mask, float* y, int B, in
 // ---------------------------------------------------------------- MaxPool2d(2) NHWC fp16 (dla_dcn.py:238)
 __global__ void maxpool2_kernel(const __half* __restrict__ x, __half* __restrict__ y, int B, int H, int W, int C,
                                 int x_ld, int y_ld) {
-  pdl_wait();
   const int Ho = H / 2, Wo = W / 2, CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Ho * Wo * CV) return;
@@ -140,7 +135,6 @@ int launch_maxpool2(const __half* x, __half* y, int B, int H, int W, int C, int 
 __global__ void upsample_add_kernel(const __half* __restrict__ x, const float* __restrict__ w,
                                     const __half* __restrict__ skip, __half* __restrict__ y, int B, int Hi, int Wi,
                                     int C, int f, int x_ld, int skip_ld, int y_ld) {
-  pdl_wait();
   const int Ho = Hi * f, Wo = Wi * f, CV = C / 8, k = 2 * f, pad = f / 2;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Ho * Wo * CV) return;
@@ -191,7 +185,6 @@ __global__ void upsample_add_kernel(const __half* __restrict__ x, const float* _
 __global__ void __launch_bounds__(256, 3)
 upsample2_add_kernel(const __half* __restrict__ x, const float* __restrict__ w, const __half* __restrict__ skip,
                      __half* __restrict__ y, int B, int Hi, int Wi, int C, int x_ld, int skip_ld, int y_ld) {
-  pdl_wait();
   const int CV = C / 8, Ho = 2 * Hi, Wo = 2 * Wi;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * (Hi + 1) * (Wi + 1) * CV) return;
@@ -271,7 +264,6 @@ int launch_upsample_add(const __half* x, const float* w, const __half* skip, __h
 __global__ void edge_gather_kernel(const __half* __restrict__ feat, int feat_ld, int ch_a, int ch_b,
                                    const long long* __restrict__ edge_idx, __half* __restrict__ ea,
                                    __half* __restrict__ eb, int B, int H, int W, int K, int out_w, int out_h) {
-  pdl_wait();
   const int CV = 32;  // 256 channels / 8
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * (K + 2) * CV * 2) return;
@@ -324,7 +316,6 @@ int launch_edge_gather(const __half* feat, int feat_ld, int ch_a, int ch_b, cons
 // with the same fp32 round trip), so that the fused head stores hidden activations for those pixels only.
 __global__ void edge_mask_kernel(const long long* __restrict__ edge_idx, unsigned char* __restrict__ mask, int B, int H,
                                  int W, int K, int out_w, int out_h) {
-  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * K) return;
   const int b = i / K;
@@ -355,7 +346,6 @@ __global__ void edge_head_add_kernel(const __half* __restrict__ t, const float* 
                                      const float* __restrict__ bias, int n_out, const long long* __restrict__ edge_idx,
                                      const long long* __restrict__ edge_len, float* __restrict__ out, int out_ctot,
                                      int out_ch0, int B, int K, int H, int W) {
-  pdl_wait();
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= B * K) return;
   const int b = warp / K, e = warp - b * K;
@@ -383,7 +373,6 @@ int launch_edge_head_add(const __half* t, const float* w, const float* bias, int
 
 // sigmoid_hm (model/layers/utils.py:39-43): x = clamp(sigmoid(x), 1e-4, 1-1e-4), in place
 __global__ void sigmoid_clamp_kernel(float* __restrict__ x, long long n) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float s = 1.f / (1.f + expf(-x[i]));
@@ -398,7 +387,6 @@ int launch_sigmoid_clamp(float* x, long long n, cudaStream_t st) {
 // out[0] += -(sum_pos log(p)(1-p)^2 + sum_neg log(1-p) p^2 (1-t)^4), out[1] += #(t==1).  (alpha=2, beta=4)
 __global__ void focal_loss_kernel(const float* __restrict__ pred, const float* __restrict__ tgt, long long n,
                                   float* __restrict__ out) {
-  pdl_wait();
   float loss = 0.f, npos = 0.f;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {

@@ -42,17 +42,10 @@ struct HeadParams {
   const unsigned char* hid_mask; // [M] or null. Non-null: only flagged pixels are stored (the ~830 border pixels per image
 };                               // the edge fusion gathers), by per-thread stores instead of a TMA store of every tile
 
-// CL = true: launched as clusters of 2 CTAs that work on two consecutive m-tiles in lock-step. Every 3x3-weight (B) box is
-// then fetched from L2 ONCE per cluster - each CTA loads 64 of its 128 rows and TMA-multicasts them into both CTAs' stage -
-// which halves the B-operand L2->SM traffic (half of this kernel's total; it is L2-bandwidth bound: 10.2 GB per B = 8
-// launch at ~12.4 TB/s). A stage is recycled only when BOTH CTAs' MMAs have released it (multicast tcgen05.commit).
-template <bool CL>
 __global__ void __launch_bounds__(320, 1)
 head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_w,
                   const __grid_constant__ CUtensorMap tmap_w2, const __grid_constant__ CUtensorMap tmap_hid,
                   const __grid_constant__ HeadParams p) {
-  pdl_launch_dependents();
-  const int crank = CL ? static_cast<int>(cluster_ctarank()) : 0;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* a_smem = smem;
@@ -81,7 +74,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
 
   if (warp == 4 && lane == 0) {
     tma_prefetch_desc(&tmap_x); tma_prefetch_desc(&tmap_w); tma_prefetch_desc(&tmap_w2); tma_prefetch_desc(&tmap_hid);
-    for (int s = 0; s < H_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], CL ? 2 : 1); }
+    for (int s = 0; s < H_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     for (int a = 0; a < 2; ++a) {
       mbar_init(&acc_full[a], 1); mbar_init(&acc_empty[a], 256);
       mbar_init(&w2_full[a], 1); mbar_init(&w2_empty[a], 1);
@@ -93,18 +86,16 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
   if (warp == 5) tmem_alloc(tmem_ptr_smem, 512);
   tc_fence_before();
   __syncthreads();
-  if (CL) cluster_sync_all();          // the peer's mbarriers are initialised before anything is multicast to them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();
 
   if (warp == 4) {
     // ================================================================ TMA producer (all lanes walk the loops, one issues)
     {
       int stage = 0, bc = 0;
       uint32_t phase = 0;
-      for (int mt = blockIdx.x; mt - crank < ntm; mt += gridDim.x) {   // CL: the pair runs the same trip count
-        const int m0 = (mt < ntm ? mt : 0) * HBM;                  // CL: an out-of-range partner tile re-reads tile 0 (discarded)
+      for (int mt = blockIdx.x; mt < ntm; mt += gridDim.x) {
+        const int m0 = mt * HBM;
         const int cn = m0 / HW, rem = m0 - cn * HW;
         const int cw = rem % p.W - 1, chh = rem / p.W - 1;          // 3x3, stride 1, pad 1
         for (int nt = 0; nt < ntn; ++nt) {
@@ -126,11 +117,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
               mbar_arrive_expect_tx(&full_bar[stage], H_ASTAGE + H_BSTAGE);
               tma_load_im2col_4d(smem_u32(a_smem + stage * H_ASTAGE), &tmap_x, &full_bar[stage], c0, cw, chh, cn,
                                  static_cast<uint16_t>(kx), static_cast<uint16_t>(ky));
-              if (CL)
-                tma_load_2d_mc(smem_u32(b_smem + stage * H_BSTAGE + crank * (HBN / 2) * 128), &tmap_w, &full_bar[stage],
-                               kb * HBK, nt * HBN + crank * (HBN / 2), static_cast<uint16_t>(3));
-              else
-                tma_load_2d(smem_u32(b_smem + stage * H_BSTAGE), &tmap_w, &full_bar[stage], kb * HBK, nt * HBN);
+              tma_load_2d(smem_u32(b_smem + stage * H_BSTAGE), &tmap_w, &full_bar[stage], kb * HBK, nt * HBN);
             }
             __syncwarp();
             c0 += HBK;
@@ -171,7 +158,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
         }
         __syncwarp();
       };
-      for (int mt = blockIdx.x; mt - crank < ntm; mt += gridDim.x) {   // CL: the pair runs the same trip count
+      for (int mt = blockIdx.x; mt < ntm; mt += gridDim.x) {
         for (int nt = 0; nt < ntn; ++nt, ++ti) {
           const int acc = ti & 1;
           mbar_wait(&acc_empty[acc], ((ti >> 1) & 1) ^ 1);
@@ -186,8 +173,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
 #pragma unroll
               for (int k4 = 0; k4 < HBK / 16; ++k4)
                 umma_f16(d_tmem, a_d0 + a_off + 2 * k4, b_d0 + b_off + 2 * k4, idesc, (kb | k4) != 0 ? 1u : 0u);
-              if (CL) umma_commit_mc(&empty_bar[stage], static_cast<uint16_t>(3));
-              else umma_commit(&empty_bar[stage]);
+              umma_commit(&empty_bar[stage]);
               if (kb == nkb - 1) umma_commit(&acc_full[acc]);
             }
             __syncwarp();
@@ -227,7 +213,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
       }
     };
     int prev_mt = 0;
-    for (int mt = blockIdx.x; mt - crank < ntm; mt += gridDim.x) {   // CL: the pair runs the same trip count
+    for (int mt = blockIdx.x; mt < ntm; mt += gridDim.x) {
       for (int nt = 0; nt < ntn; ++nt, ++ti) {
         const int acc = ti & 1, br = nt >> 1, n0 = nt * HBN;
         if (store_pending && et == 0) bulk_wait_read0();
@@ -301,7 +287,6 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_const
   }
   tc_fence_before();
   __syncthreads();
-  if (CL) cluster_sync_all();          // no CTA leaves while its peer may still multicast into it
   if (warp == 5) tmem_dealloc(tmem_base, 512);
 }
 
@@ -362,33 +347,19 @@ int launch_head_fused(const __half* x, int x_ld, int B, int H, int W, int Cin, c
                CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
   };
   const int K3 = 9 * Cin;
-  const bool cl = g_tunable[9] != 0;                       // 2-CTA clusters with multicast weight loads
-  if (!tiled2d(&tw, w3, K3, nbranch * 256, K3, 64, cl ? HBN / 2 : HBN) || !tiled2d(&tw2, w2, 256, nbranch * 32, 256, 64, 32) ||
+  if (!tiled2d(&tw, w3, K3, nbranch * 256, K3, 64, HBN) || !tiled2d(&tw2, w2, 256, nbranch * 32, 256, 64, 32) ||
       !tiled2d(&th, hid, hid_ld, p.M, hid_ld, 64, HBM)) { set_error("head_fused: tiled tensor map failed"); return -1; }
   static bool attr = false;
   if (!attr) {
-    if (check_cuda(cudaFuncSetAttribute(head_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, H_SMEM), "head smem")) return -1;
-    if (check_cuda(cudaFuncSetAttribute(head_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, H_SMEM), "head smem")) return -1;
+    if (check_cuda(cudaFuncSetAttribute(head_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, H_SMEM), "head smem")) return -1;
     attr = true;
   }
   int dev = 0, nsm = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
   const int ntm = (p.M + HBM - 1) / HBM;
-  if (!cl) {
-    const int grid = ntm < nsm ? ntm : nsm;
-    return check_cuda(launch_k(head_fused_kernel<false>, dim3(grid), dim3(320), H_SMEM, st, tx, tw, tw2, th, p), "head_fused launch");
-  }
-  int grid = (ntm + 1) & ~1;                               // whole pairs; an odd last tile gets an all-out-of-range partner
-  if (grid > (nsm & ~1)) grid = nsm & ~1;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(320); cfg.dynamicSmemBytes = H_SMEM; cfg.stream = st;
-  cudaLaunchAttribute la[1];
-  la[0].id = cudaLaunchAttributeClusterDimension;
-  la[0].val.clusterDim.x = 2; la[0].val.clusterDim.y = 1; la[0].val.clusterDim.z = 1;
-  cfg.attrs = la; cfg.numAttrs = 1;
-  return check_cuda(cudaLaunchKernelEx(&cfg, head_fused_kernel<true>, tx, tw, tw2, th, p), "head_fused cluster launch");
+  const int grid = ntm < nsm ? ntm : nsm;
+  return check_cuda(launch_k(head_fused_kernel, dim3(grid), dim3(320), H_SMEM, st, tx, tw, tw2, th, p), "head_fused launch");
 }
 
 }  // namespace mf

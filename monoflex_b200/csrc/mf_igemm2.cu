@@ -25,33 +25,17 @@ static constexpr int BM = 128;
 static constexpr int BK = 64;
 static constexpr int A_STAGE = BM * BK * 2;   // 16 KB
 
-static constexpr int AS_MAX_KB = 9;          // A-stationary mode: at most 9 resident K blocks (3x3 taps of 64 channels)
-
-// MODE_CONV_PATCH (3x3, stride 1, pad 1, Cin % 64 == 0): an m-tile is a 16 x 8 pixel patch (as in MODE_DCN) and the A operand
-// is NOT fetched tap by tap. Per 64-channel chunk (and per hi / lo half) three "slots" are loaded, one per kx: the tiled TMA box
-// {64 ch, 16 px, 10 rows} at x0 + kx - 1, y0 - 1 (zero fill outside the image = the conv padding). A slot is 160 rows of
-// 128 B in the 128B-swizzle layout, so the A tile of tap (ky, kx) is the 128 rows starting ky * 16 rows = ky * 2048 B into
-// slot kx - a multiple of the 1024 B swizzle period, i.e. just another descriptor start address. 60 KB of A per chunk instead
-// of nine 16 KB im2col boxes (144 KB): these layers are bound by L2 -> smem operand traffic (ncu: 11.7 TB/s of TMA reads on
-// the predictor GEMM, the chip's L2 limit), not by the tensor pipe.
-static constexpr int PATCH_SLOT = 10 * 16 * 128;     // 20 KB
-
 // SPLIT: the fp16 NHWC output is a hi/lo pair (strict-precision mode): two staging tiles per 64-channel sub-tile, paid for
 // with one pipeline stage (the K loop of a split layer is 3x longer, so the shallower ring costs nothing measurable).
-// EPI (see igemm2_kernel): 1 = SPLIT doubles the staging, 2 = HEAD2 has no output staging at all (256-column tiles fit).
+// EPI (see igemm2_kernel): 1 = SPLIT doubles the staging, 2 = HEAD2 has no output staging at all.
 template <int BLOCK_N, int MODE, int EPI = 0>
 struct Cfg2 {
   static constexpr bool SPLIT = EPI == 1;
-  static constexpr bool A_STAT = MODE == MODE_CONV_TMA_AS;
-  static constexpr bool PATCH = MODE == MODE_CONV_PATCH;
-  // patch mode: ring of A slots + ring of weight stages (one stage = the BLOCK_N x 64 block of one tap / chunk / half)
-  static constexpr int NSLOT = !PATCH ? 0 : (BLOCK_N >= 128 ? (EPI == 2 ? 6 : 4) : (BLOCK_N >= 64 ? 6 : 8));
-  static constexpr int PSTAGES = BLOCK_N >= 128 ? (EPI == 2 ? 6 : 4) : (BLOCK_N >= 64 ? 6 : 8);
-  static constexpr int STAGES0 = PATCH ? PSTAGES : A_STAT ? 3 : (MODE == MODE_DCN ? 4 : (BLOCK_N >= 256 ? 4 : BLOCK_N >= 128 ? 5 : (BLOCK_N >= 64 ? 6 : (BLOCK_N >= 32 ? 5 : 6))));
-  static constexpr int STAGES = PATCH ? STAGES0 : (SPLIT && BLOCK_N >= 64) ? ((MODE == MODE_DCN && BLOCK_N < 128) ? STAGES0 : STAGES0 - 1) : STAGES0;
-  static constexpr int A_REGION = PATCH ? NSLOT * PATCH_SLOT : (A_STAT ? AS_MAX_KB : STAGES) * A_STAGE;
+  static constexpr int STAGES0 = MODE == MODE_DCN ? 4 : (BLOCK_N >= 128 ? 5 : (BLOCK_N >= 64 ? 6 : (BLOCK_N >= 32 ? 5 : 6)));
+  static constexpr int STAGES = (SPLIT && BLOCK_N >= 64) ? ((MODE == MODE_DCN && BLOCK_N < 128) ? STAGES0 : STAGES0 - 1) : STAGES0;
+  static constexpr int A_REGION = STAGES * A_STAGE;
   static constexpr int LAG = BLOCK_N >= 64 ? 3 : (BLOCK_N >= 32 ? 3 : 4);   // cp.async groups in flight per producer thread
-  static constexpr int CTAS_PER_SM = (BLOCK_N >= 64 || PATCH) ? 1 : 2;
+  static constexpr int CTAS_PER_SM = BLOCK_N >= 64 ? 1 : 2;
   static constexpr int B_STAGE = BLOCK_N * BK * 2;
   static constexpr int OUT_HALF = BLOCK_N >= 64 ? (BLOCK_N / 64) * A_STAGE : 0;     // staging of one fp16 tile
   static constexpr int OUT_STAGE = EPI == 2 ? 0 : (SPLIT ? 2 * OUT_HALF : OUT_HALF);
@@ -79,20 +63,16 @@ MF_DEVINL void act_chunk(float (&v)[N], int act, int nb) {
 
 // EPI: 0 = plain epilogue, 1 = SPLIT (staged hi/lo output tiles), 2 = HEAD2 (1x1 head contraction in the epilogue, see IgemmParams)
 template <int BLOCK_N, int MODE, int NPW, int EPI>
-__global__ void __launch_bounds__((NPW + (MODE == MODE_CONV_PATCH ? 7 : 6)) * 32, Cfg2<BLOCK_N, MODE, EPI>::CTAS_PER_SM)
+__global__ void __launch_bounds__((NPW + 6) * 32, Cfg2<BLOCK_N, MODE, EPI>::CTAS_PER_SM)
 igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_y,
               const __grid_constant__ CUtensorMap tmap_x, const IgemmParams p, const int use_tma_store) {
-  constexpr bool PATCH = (MODE == MODE_CONV_PATCH);     // 16 x 8 pixel m-tiles, A from kx-shifted patch slots (see PATCH_SLOT)
-  constexpr bool PTILE = (MODE == MODE_DCN || PATCH);   // m-tile = 16 x 8 patch of one image
-  constexpr bool A_TMA = (MODE == MODE_CONV_TMA || MODE == MODE_CONV_TMA_AS || PATCH);
-  constexpr bool A_STAT = (MODE == MODE_CONV_TMA_AS);   // A tile of an m-tile stays resident while all n-tiles stream B
-  constexpr bool M_OUTER = A_STAT || PATCH;             // tile enumeration: m-tile strided over CTAs, n-tiles inside
+  constexpr bool PTILE = (MODE == MODE_DCN);            // m-tile = 16 x 8 patch of one image
+  constexpr bool A_TMA = (MODE == MODE_CONV_TMA);
   constexpr int EPI_THREADS = A_TMA ? 128 + NPW * 32 : 128;
   constexpr bool SPLIT = EPI == 1;
   constexpr bool HEAD2 = EPI == 2;
   using C = Cfg2<BLOCK_N, MODE, EPI>;
   constexpr int STAGES = C::STAGES;
-  constexpr int NSL = Cfg2<BLOCK_N, MODE, EPI>::NSLOT > 0 ? Cfg2<BLOCK_N, MODE, EPI>::NSLOT : 1;      // patch-mode A slots
   constexpr int LAG = C::LAG;
   const bool split_out = SPLIT || p.split_out != 0;      // SPLIT == staged hi/lo tiles; narrow tiles store both halves directly
   constexpr int B_STAGE = C::B_STAGE;
@@ -100,7 +80,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
   constexpr int RPP = NPT / 8;
   constexpr int PASSES = BM / RPP;
 
-  pdl_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* a_smem = smem;
@@ -110,9 +89,7 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
   uint64_t* empty_bar = full_bar + STAGES;
   uint64_t* acc_full = empty_bar + STAGES;     // [2]
   uint64_t* acc_empty = acc_full + 2;          // [2]
-  uint64_t* a_full = acc_empty + 2;            // [AS_MAX_KB]  (A-stationary mode)
-  uint64_t* a_empty = a_full + AS_MAX_KB;      // [AS_MAX_KB]  ([0] only in A-stationary mode; one per slot in patch mode)
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(a_empty + AS_MAX_KB);
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(acc_empty + 2);
   float* sc_s = reinterpret_cast<float*>(o_smem + C::OUT_STAGE + C::BAR_BYTES);
   float* sh_s = sc_s + BLOCK_N;
   uint8_t* prm_smem = reinterpret_cast<uint8_t*>(sh_s + BLOCK_N);      // MODE_DCN only: 9*128 sampling records (36 KB)
@@ -124,16 +101,7 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
   const int ntm = PTILE ? p.B * tiles_x * tiles_y : (p.M + BM - 1) / BM;
   const int ntiles = ntn * ntm;
   const int nkb = p.nkb;
-  // tile enumeration: plain = tile t, t += grid (n fastest); A-stationary = m-tile outer (strided over CTAs), n inner
-  const int n_outer = M_OUTER ? ntm : ntiles, n_inner = M_OUTER ? ntn : 1;
-#define MF_TILE_LOOP                                                         \
-  for (int outer = blockIdx.x; outer < n_outer; outer += gridDim.x)          \
-    for (int inner = 0; inner < n_inner; ++inner)
-#define MF_TILE_INDEX (M_OUTER ? outer * ntn + inner : outer)
   const int HoWo = p.Ho * p.Wo;
-  // patch mode: 64-channel chunks, hi / lo halves, and whether the A slots of an m-tile stay resident over its n-tiles
-  const int p_nchunk = p.Cin >> 6, p_nh = p.split_in ? 2 : 1;
-  const bool p_stat = PATCH && p_nchunk == 1 && ntn > 1 && 3 * p_nh <= NSL;
 
   if (warp == NPW && lane == 0) {
     tma_prefetch_desc(&tmap_w);
@@ -147,7 +115,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
       mbar_init(&acc_full[a], 1);
       mbar_init(&acc_empty[a], EPI_THREADS);
     }
-    for (int a = 0; a < AS_MAX_KB; ++a) { mbar_init(&a_full[a], 1); mbar_init(&a_empty[a], 1); }
     fence_mbar_init();
   }
   if (warp == NPW + 1) tmem_alloc(tmem_ptr_smem, C::TMEM_COLS);
@@ -155,7 +122,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();            // everything above overlapped the previous kernel's tail; from here on we touch its outputs
 
   // ================================================================ epilogue body (run by 1 or 2 warp groups)
   auto run_epilogue = [&](const int group, const int et) {
@@ -167,9 +133,8 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
     const bool staged = use_tma_store != 0;             // host guarantees OUT_F16_NHWC && BLOCK_N >= 64
     const uint32_t sc_u = smem_u32(sc_s), sh_u = smem_u32(sh_s), o_u = smem_u32(o_smem);
     int ti = -1;
-    MF_TILE_LOOP {
+    for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
       ++ti;
-      const int t = MF_TILE_INDEX;
       const int acc = ti & 1;
       const int n0 = (t % ntn) * BLOCK_N;
       const int m_tile = t / ntn;
@@ -502,9 +467,9 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
         for (int q = 0; q < PASSES; ++q) dst_off[q] = sw128_off(q * RPP + rsub, j);
         if constexpr (SPLIT) {
           // strict precision: hi and lo halves of the four corners are blended in fp32 ONCE per (tap, 64-channel chunk) and
-          // feed three consecutive K blocks: hi (x W_hi), lo (x W_hi), hi again (x W_lo).
+          // fill the two stages of the pair schedule (see IgemmParams::pair): hi, then lo.
           const int lo_bytes = p.x_lo * 2;
-          for (int kb = 0; kb < nkb; kb += (p.pair ? 2 : 3)) {
+          for (int kb = 0; kb < nkb; kb += 2) {
             const char* xb = x_img + c0 * 2;
             const uint32_t rec = (tap * BM + rsub) * 16;
             uint4 hi4[PASSES], lo4[PASSES];
@@ -550,8 +515,7 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
               }
             }
 #pragma unroll
-            for (int which = 0; which < 3; ++which) {
-              if (which == 2 && p.pair) break;               // pair schedule: the MMA warp re-uses the hi stage for A_hi W_lo
+            for (int which = 0; which < 2; ++which) {
               mbar_wait(&empty_bar[stage], phase ^ 1);
               const uint32_t a_stage = smem_u32(a_smem + stage * A_STAGE);
 #pragma unroll
@@ -610,66 +574,16 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
         }
       }
     }
-  } else if (warp == NPW && PATCH) {
-    // ================================================================ patch mode: this warp streams the weight stages ...
+  } else if (warp == NPW) {
+    // ================================================================ weight tiles (and MODE_CONV_TMA A boxes) by TMA (all
+    // lanes walk, one issues)
     {
       int stage = 0;
       uint32_t phase = 0;
-      MF_TILE_LOOP {
-        const int n0 = inner * BLOCK_N;
-        for (int c = 0; c < p_nchunk; ++c)
-          for (int kx = 0; kx < 3; ++kx)
-            for (int ky = 0; ky < 3; ++ky) {
-              const int g = (ky * 3 + kx) * p_nchunk + c;          // (tap, chunk) group of the packed weight K axis
-              for (int h = 0; h < p_nh; ++h) {
-                mbar_wait(&empty_bar[stage], phase ^ 1);
-                if (elect_one()) {
-                  mbar_arrive_expect_tx(&full_bar[stage], B_STAGE);
-                  tma_load_2d(smem_u32(b_smem + stage * B_STAGE), &tmap_w, &full_bar[stage], (p.split_in ? 3 * g + 2 * h : g) * BK, n0);
-                }
-                __syncwarp();
-                if (++stage == STAGES) { stage = 0; phase ^= 1; }
-              }
-            }
-      }
-    }
-  } else if (PATCH && warp == NPW + 6) {
-    // ================================================================ ... and an extra warp the A slots: two independent
-    // in-order producers (in one warp the two wait loops would serialise: a try_wait suspends the whole warp)
-    {
-      int fa = 0;                                                  // running slot-fill counter: slot fa % NSLOT
-      for (int outer = blockIdx.x; outer < n_outer; outer += gridDim.x) {
-        const int tile_b = outer / (tiles_x * tiles_y);
-        const int tile_t = outer - tile_b * (tiles_x * tiles_y);
-        const int y0 = (tile_t / tiles_x) << 3, x0 = (tile_t % tiles_x) << 4;
-        const int reps = p_stat ? 1 : n_inner;
-        for (int rp = 0; rp < reps; ++rp)
-          for (int c = 0; c < p_nchunk; ++c)
-            for (int kx = 0; kx < 3; ++kx)
-              for (int h = 0; h < p_nh; ++h) {
-                const int s = fa % NSL;
-                mbar_wait(&a_empty[s], (((fa / NSL) & 1) ^ 1));
-                if (elect_one()) {
-                  mbar_arrive_expect_tx(&a_full[s], PATCH_SLOT);
-                  tma_load_4d(smem_u32(a_smem + s * PATCH_SLOT), &tmap_x, &a_full[s], c * 64 + (h ? p.x_lo : 0), x0 + kx - 1, y0 - 1,
-                              tile_b);
-                }
-                __syncwarp();
-                ++fa;
-              }
-      }
-    }
-  } else if (warp == NPW) {
-    // ================================================================ weight tiles by TMA (all lanes walk, one issues)
-    {
-      int stage = 0, mi = 0;
-      uint32_t phase = 0;
-      const int kc = A_TMA ? p.kc : BK, nbox = BK / kc, box_bytes = BM * kc * 2, ntap = p.kh * p.kw;
-      MF_TILE_LOOP {
-        const int t = MF_TILE_INDEX;
+      for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
         const int n0 = (t % ntn) * BLOCK_N;
         int cw = 0, chh = 0, cn = 0;
-        if (A_TMA && (!A_STAT || inner == 0)) {   // coordinates of the tile's first output pixel in input space (incl. -pad)
+        if (A_TMA) {                                    // coordinates of the tile's first output pixel in input space (incl. -pad)
           const int m0 = (t / ntn) * BM;
           cn = m0 / HoWo;
           const int rem = m0 - cn * HoWo;
@@ -677,40 +591,21 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
           cw = ox * p.stride - p.pad;
           chh = oy * p.stride - p.pad;
         }
-        if (A_STAT && inner == 0) {               // the whole A tile (all taps) once per m-tile, one barrier per K block
-          mbar_wait(a_empty, (mi & 1) ^ 1);
-          ++mi;
-          int tap = 0, c0 = 0, kx = 0, ky = 0;
-          for (int kb = 0; kb < nkb; ++kb) {
-            if (elect_one()) {
-              mbar_arrive_expect_tx(&a_full[kb], A_STAGE);
-              tma_load_im2col_4d(smem_u32(a_smem + kb * A_STAGE), &tmap_x, &a_full[kb], c0, cw, chh, cn,
-                                 static_cast<uint16_t>(kx), static_cast<uint16_t>(ky));
-            }
-            __syncwarp();
-            c0 += BK;
-            if (c0 >= p.Cin) { c0 = 0; ++tap; if (++kx == p.kw) { kx = 0; ++ky; } }
-          }
-        }
-        int tap = 0, c0 = 0, kx = 0, ky = 0;            // running (tap, channel) cursor: no divisions in the K loop
-        int which = 0;                                  // split_in: 0 = A_hi W_hi, 1 = A_lo W_hi, 2 = A_hi W_lo (same A box as 0)
+        int c0 = 0, kx = 0, ky = 0;                     // running (tap, channel) cursor: no divisions in the K loop
+        int which = 0;                                  // split_in: 0 = A_hi box, 1 = A_lo box of the same (tap, chunk)
         for (int kb = 0; kb < nkb; ++kb) {
           mbar_wait(&empty_bar[stage], phase ^ 1);
           const bool issuer = elect_one();
-          if (issuer) mbar_arrive_expect_tx(&full_bar[stage], (A_TMA && !A_STAT) ? A_STAGE + B_STAGE : B_STAGE);
-          if (A_TMA && !A_STAT) {
-            const uint32_t a_dst = smem_u32(a_smem + stage * A_STAGE);
-            for (int jb = 0; jb < nbox; ++jb) {
-              const bool valid = tap < ntap;              // K tail: channel coordinate out of range -> TMA zero fill
-              if (issuer)
-                tma_load_im2col_4d(a_dst + jb * box_bytes, &tmap_x, &full_bar[stage],
-                                   valid ? c0 + (which == 1 ? p.x_lo : 0) : p.Cin, cw, chh, cn,
-                                   static_cast<uint16_t>(valid ? kx : 0), static_cast<uint16_t>(valid ? ky : 0));
-              if (p.split_in && ++which < (p.pair ? 2 : 3)) continue;
+          if (issuer) mbar_arrive_expect_tx(&full_bar[stage], A_TMA ? A_STAGE + B_STAGE : B_STAGE);
+          if (A_TMA) {
+            if (issuer)
+              tma_load_im2col_4d(smem_u32(a_smem + stage * A_STAGE), &tmap_x, &full_bar[stage], c0 + (which == 1 ? p.x_lo : 0),
+                                 cw, chh, cn, static_cast<uint16_t>(kx), static_cast<uint16_t>(ky));
+            if (!p.split_in || ++which == 2) {
               which = 0;
-              c0 += kc;
+              c0 += BK;
               if (c0 >= p.Cin) {
-                c0 = 0; ++tap;
+                c0 = 0;
                 if (++kx == p.kw) { kx = 0; ++ky; }
               }
             }
@@ -734,79 +629,16 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
       uint64_t a_d0[BK / 16];
       const uint32_t a0 = smem_u32(a_smem), b0 = smem_u32(b_smem);
 #pragma unroll
-      for (int k4 = 0; k4 < BK / 16; ++k4) {
-        if (!A_TMA || p.kc == 64) a_d0[k4] = umma_desc_sw128(a0 + k4 * 32);
-        else if (p.kc == 32) a_d0[k4] = umma_desc_kmajor(a0 + (k4 >> 1) * (BM * 64) + (k4 & 1) * 32, 16, 512, 4);
-        else if (p.kc == 16) a_d0[k4] = umma_desc_kmajor(a0 + k4 * (BM * 32), 16, 256, 6);
-        else a_d0[k4] = umma_desc_kmajor(a0 + k4 * (2 * BM * 16), BM * 16, 128, 0);       // kc == 8: two boxes per MMA
-      }
+      for (int k4 = 0; k4 < BK / 16; ++k4) a_d0[k4] = umma_desc_sw128(a0 + k4 * 32);
       const uint64_t b_d0 = umma_desc_sw128(b0);
-      int stage = 0, ti = -1, mi = -1;
-      int fa = 0, fa_base = 0;                                       // patch mode: slot-fill counter (as in the A producer)
+      int stage = 0, ti = -1;
       uint32_t phase = 0;
-      MF_TILE_LOOP {
+      for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
         ++ti;
-        if (inner == 0) ++mi;
         const int acc = ti & 1;
         mbar_wait(&acc_empty[acc], ((ti >> 1) & 1) ^ 1);          // epilogue has drained this accumulator
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + acc * C::ACC_COLS;
-        if constexpr (PATCH) {
-          if (inner == 0) fa_base = fa;
-          if (p_stat) fa = fa_base;                                  // the resident slots of this m-tile, again
-          uint32_t accum = 0;
-          for (int c = 0; c < p_nchunk; ++c)
-            for (int kx = 0; kx < 3; ++kx) {
-              const int s_hi = fa % NSL;
-              mbar_wait(&a_full[s_hi], (fa / NSL) & 1);
-              ++fa;
-              int s_lo = s_hi;
-              if (p_nh == 2) {
-                s_lo = fa % NSL;
-                mbar_wait(&a_full[s_lo], (fa / NSL) & 1);
-                ++fa;
-              }
-              tc_fence_after();
-              for (int ky = 0; ky < 3; ++ky) {
-                const uint64_t a_hi = static_cast<uint64_t>((s_hi * PATCH_SLOT + ky * 2048) >> 4);
-                const uint64_t a_lo = static_cast<uint64_t>((s_lo * PATCH_SLOT + ky * 2048) >> 4);
-                const int s0 = stage;
-                mbar_wait(&full_bar[s0], phase);
-                tc_fence_after();
-                const uint64_t b0s = static_cast<uint64_t>((s0 * B_STAGE) >> 4);
-                if (elect_one()) {
-#pragma unroll
-                  for (int k4 = 0; k4 < BK / 16; ++k4)                               // A_hi W_hi (or the only product)
-                    umma_f16(d_tmem, a_d0[k4] + a_hi, b_d0 + b0s + 2 * k4, idesc, k4 == 0 ? accum : 1u);
-                  if (p_nh == 1) umma_commit(&empty_bar[s0]);
-                }
-                __syncwarp();
-                accum = 1u;
-                if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                if (p_nh == 2) {
-                  const int s1 = stage;
-                  mbar_wait(&full_bar[s1], phase);
-                  tc_fence_after();
-                  const uint64_t b1s = static_cast<uint64_t>((s1 * B_STAGE) >> 4);
-                  if (elect_one()) {
-#pragma unroll
-                    for (int k4 = 0; k4 < BK / 16; ++k4) umma_f16(d_tmem, a_d0[k4] + a_lo, b_d0 + b0s + 2 * k4, idesc, 1u);   // A_lo W_hi
-#pragma unroll
-                    for (int k4 = 0; k4 < BK / 16; ++k4) umma_f16(d_tmem, a_d0[k4] + a_hi, b_d0 + b1s + 2 * k4, idesc, 1u);   // A_hi W_lo
-                    umma_commit(&empty_bar[s0]);
-                    umma_commit(&empty_bar[s1]);
-                  }
-                  __syncwarp();
-                  if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                }
-              }
-              if ((!p_stat || inner == n_inner - 1) && elect_one()) {   // last reader of these slots
-                umma_commit(&a_empty[s_hi]);
-                if (p_nh == 2) umma_commit(&a_empty[s_lo]);
-              }
-              __syncwarp();
-            }
-        } else
         if (p.pair) {
           // pair schedule: stage s0 = (A_hi, W_hi), stage s1 = (A_lo, W_lo) of one (tap, 64-channel chunk); three products
           for (int kb = 0; kb < nkb; kb += 2) {
@@ -840,10 +672,9 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
           }
         } else
         for (int kb = 0; kb < nkb; ++kb) {
-          if (A_STAT && inner == 0) mbar_wait(&a_full[kb], mi & 1);   // resident A block of this m-tile has landed
           mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
-          const uint64_t a_off = static_cast<uint64_t>(((A_STAT ? kb : stage) * A_STAGE) >> 4);
+          const uint64_t a_off = static_cast<uint64_t>((stage * A_STAGE) >> 4);
           const uint64_t b_off = static_cast<uint64_t>((stage * B_STAGE) >> 4);
           if (elect_one()) {
 #pragma unroll
@@ -855,10 +686,7 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
           __syncwarp();
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
-        if (elect_one()) {
-          umma_commit(&acc_full[acc]);
-          if (A_STAT && inner == n_inner - 1) umma_commit(a_empty);   // every MMA reading the resident A tile is done
-        }
+        if (elect_one()) umma_commit(&acc_full[acc]);
         __syncwarp();
       }
     }
@@ -927,27 +755,21 @@ static int launch2_cfg(const CUtensorMap& tw, const CUtensorMap& ty, const CUten
                        int use_tma_store, cudaStream_t st) {
   using C = Cfg2<BLOCK_N, MODE, EPI>;
   auto kern = igemm2_kernel<BLOCK_N, MODE, NPW, EPI>;
-  static int attr_smem = 0;
-  int smem = C::SMEM + g_tunable[MODE == MODE_DCN ? 0 : 1];
-  if (smem > 227 * 1024) smem = 227 * 1024;
-  if (smem > attr_smem) {
-    if (check_cuda(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem), "smem attr")) return -1;
-    attr_smem = smem;
+  static bool attr_set = false;
+  if (!attr_set) {
+    if (check_cuda(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM), "smem attr")) return -1;
+    attr_set = true;
   }
   const int ntn = (p.Cout + BLOCK_N - 1) / BLOCK_N;
-  const int ntm = (MODE == MODE_DCN || MODE == MODE_CONV_PATCH) ? p.B * ((p.H + 7) / 8) * ((p.W + 15) / 16) : (p.M + BM - 1) / BM;
+  const int ntm = MODE == MODE_DCN ? p.B * ((p.H + 7) / 8) * ((p.W + 15) / 16) : (p.M + BM - 1) / BM;
   int grid = num_sms() * C::CTAS_PER_SM;
   if (grid > ntn * ntm) grid = ntn * ntm;
-  if (MODE == MODE_CONV_PATCH && grid > ntm) grid = ntm;       // m-tiles are strided over CTAs, n-tiles run inside
-  return check_cuda(launch_k(kern, dim3(grid), dim3((NPW + (MODE == MODE_CONV_PATCH ? 7 : 6)) * 32), smem, st, tw, ty, tx, p,
-                             use_tma_store),
-                    "igemm2 launch");
+  return check_cuda(launch_k(kern, dim3(grid), dim3((NPW + 6) * 32), C::SMEM, st, tw, ty, tx, p, use_tma_store), "igemm2 launch");
 }
 
 // out[b, ch, pix] = bias[ch] + sum over the eight partial planes (fixed order: deterministic), ch < ncls -> cls, else reg
 __global__ void head2_reduce_kernel(const float* __restrict__ part, const float* __restrict__ bias, float* __restrict__ cls,
                                     float* __restrict__ reg, int B, int ncls, int nreg, int HW) {
-  pdl_wait();
   const int ntot = ncls + nreg;
   const long long plane = static_cast<long long>(B) * ntot * HW;
   const long long i = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) * 4;
@@ -979,18 +801,9 @@ int launch_head2_reduce(const float* part, const float* bias, float* cls, float*
 int launch_igemm2(const IgemmParams& p, const __half* wp, int n_pad, int k_pad, int mode, cudaStream_t st) {
   PFN_encodeTiled2 enc = encode_fn();
   if (!enc) return -1;
-  // patch mode (see PATCH_SLOT): 3x3 / stride 1 / pad 1 layers on pair input whose maps tile exactly into 16 x 8 patches.
-  // Opt-in (tunable 13 / MF_PATCH=1): measured SLOWER than the im2col boxes at B = 8 (offset convs 0.75 vs 0.64 ms, base
-  // convs 1.71 vs 1.64 ms, predictor 1.55 vs 1.39 ms) although it moves half the bytes - kept as a tested experiment.
-  const bool patch_geom = mode == MODE_CONV && p.split_in && p.kh == 3 && p.kw == 3 && p.stride == 1 && p.pad == 1 &&
-                          p.Cin % 64 == 0 && p.H % 8 == 0 && p.W % 16 == 0 && g_tunable[13] == 1 && g_tunable[4] == 0 &&
-                          (reinterpret_cast<uintptr_t>(p.x) & 15) == 0 && p.x_ld % 8 == 0;
-  // HEAD2 tiles: 128 columns (1.39 ms at B = 8); 256-column tiles (tunable 12) measured 1.56 ms once the MMA issue was fixed
-  const int bn = p.h2_w != nullptr ? ((patch_geom || g_tunable[12] == 0) ? 128 : 256) : igemm_block_n(p.Cout);
-  const bool store_ok = p.out_mode == OUT_F16_NHWC && bn >= 64 && g_tunable[3] == 0 &&
-                        (reinterpret_cast<uintptr_t>(p.y) & 15) == 0 && p.y_ld % 8 == 0;
-  const bool patch = patch_geom && (p.h2_w != nullptr || (p.split_out && store_ok && (bn == 64 || bn == 128)) ||
-                                    (!p.split_out && p.out_mode == OUT_F32_NHWC && bn == 32));
+  // HEAD2 tiles: 128 columns (1.39 ms at B = 8; 256-column tiles measured 1.56 ms)
+  const int bn = p.h2_w != nullptr ? 128 : igemm_block_n(p.Cout);
+  const bool store_ok = p.out_mode == OUT_F16_NHWC && bn >= 64 && (reinterpret_cast<uintptr_t>(p.y) & 15) == 0 && p.y_ld % 8 == 0;
   if (n_pad % bn != 0 || k_pad % BK != 0 || k_pad < p.nkb * BK) {
     set_error("igemm: packed weight shape [%d,%d] incompatible with block_n=%d nkb=%d", n_pad, k_pad, bn, p.nkb);
     return -1;
@@ -1030,7 +843,7 @@ int launch_igemm2(const IgemmParams& p, const __half* wp, int n_pad, int k_pad, 
   ty = tw;
   if (store_ok) {
     CUresult r;
-    if (mode == MODE_DCN || patch) {
+    if (mode == MODE_DCN) {
       cuuint64_t gdim[4] = {static_cast<cuuint64_t>(p.Cout + (p.split_out ? p.y_lo : 0)), static_cast<cuuint64_t>(p.W),
                             static_cast<cuuint64_t>(p.H), static_cast<cuuint64_t>(p.B)};
       cuuint64_t gstr[3] = {static_cast<cuuint64_t>(p.y_ld) * 2, static_cast<cuuint64_t>(p.y_ld) * 2 * p.W,
@@ -1050,34 +863,14 @@ int launch_igemm2(const IgemmParams& p, const __half* wp, int n_pad, int k_pad, 
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(output) failed (%d)", static_cast<int>(r)); return -1; }
     use_tma_store = 1;
   }
-  // A operand by im2col-mode TMA whenever a K block is one (tap, 64-channel) box
+  // A operand by im2col-mode TMA whenever a K block is one (tap, 64-channel) box. Narrower boxes (Cin 8 / 16 / 32) are
+  // request-bound inside the TMA unit (measured: the 7x7 stem 1.8x slower than the cp.async gather), so those layers stay on
+  // the gather producers.
   CUtensorMap tx = tw;
   bool a_tma = false;
   IgemmParams pp = p;
-  const int kc = p.Cin % 64 == 0 ? 64 : p.Cin;
-  if (p.split_in && kc != 64 && g_tunable[5] != 0) { set_error("igemm: small-C im2col TMA is not built for split input"); return -1; }
-  // im2col boxes narrower than 128 B are request-bound inside the TMA unit (measured: the 7x7 stem 1.8x slower than the
-  // cp.async gather), so they stay on the gather producers unless tunable 5 asks for them.
-  if (patch) {
-    cuuint64_t gdim[4] = {static_cast<cuuint64_t>(p.Cin + p.x_lo), static_cast<cuuint64_t>(p.W), static_cast<cuuint64_t>(p.H),
-                          static_cast<cuuint64_t>(p.B)};
-    cuuint64_t gstr[3] = {static_cast<cuuint64_t>(p.x_ld) * 2, static_cast<cuuint64_t>(p.x_ld) * 2 * p.W,
-                          static_cast<cuuint64_t>(p.x_ld) * 2 * p.W * p.H};
-    cuuint32_t box[4] = {64, 16, 10, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<__half*>(p.x), gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(patch input) failed (%d)", static_cast<int>(r)); return -1; }
-    pp.kc = 64;
-    pp.pair = 1;
-    if (p.h2_w != nullptr) return launch2_cfg<128, MODE_CONV_PATCH, 4, 2>(tw, ty, tx, pp, 0, st);
-    if (bn == 32) return launch2_cfg<32, MODE_CONV_PATCH, 4, 0>(tw, ty, tx, pp, 0, st);
-    if (bn == 64) return launch2_cfg<64, MODE_CONV_PATCH, 4, 1>(tw, ty, tx, pp, use_tma_store, st);
-    return launch2_cfg<128, MODE_CONV_PATCH, 4, 1>(tw, ty, tx, pp, use_tma_store, st);
-  }
-  if (mode == MODE_CONV && (kc == 64 || ((kc == 32 || kc == 16 || kc == 8) && g_tunable[5] != 0)) && g_tunable[4] == 0 &&
-      (reinterpret_cast<uintptr_t>(p.x) & 15) == 0 && p.kw <= 16 && p.kh <= 16 && p.stride <= 8) {
+  if (mode == MODE_CONV && p.Cin % 64 == 0 && (reinterpret_cast<uintptr_t>(p.x) & 15) == 0 && p.kw <= 16 && p.kh <= 16 &&
+      p.stride <= 8) {
     PFN_encodeIm2col enc2 = encode_im2col_fn();
     if (!enc2) return -1;
     cuuint64_t gdim[4] = {static_cast<cuuint64_t>(p.Cin + (p.split_in ? p.x_lo : 0)), static_cast<cuuint64_t>(p.W),
@@ -1087,27 +880,21 @@ int launch_igemm2(const IgemmParams& p, const __half* wp, int n_pad, int k_pad, 
     int lower[2] = {-p.pad, -p.pad};
     int upper[2] = {p.pad - (p.kw - 1), p.pad - (p.kh - 1)};
     cuuint32_t estr[4] = {1, static_cast<cuuint32_t>(p.stride), static_cast<cuuint32_t>(p.stride), 1};
-    const CUtensorMapSwizzle sw = kc == 64 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                  : kc == 32 ? CU_TENSOR_MAP_SWIZZLE_64B
-                                  : kc == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE;
-    CUresult r = enc2(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<__half*>(p.x), gdim, gstr, lower, upper,
-                      static_cast<cuuint32_t>(kc), BM, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                      CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeIm2col failed (%d) kc=%d", static_cast<int>(r), kc); return -1; }
+    CUresult r = enc2(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<__half*>(p.x), gdim, gstr, lower, upper, BK, BM, estr,
+                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeIm2col failed (%d)", static_cast<int>(r)); return -1; }
     a_tma = true;
-    pp.kc = kc;
   }
-  if (p.split_in && g_tunable[11] == 0 && (mode == MODE_DCN || (a_tma && kc == 64))) {
+  if (p.split_in && (mode == MODE_DCN || a_tma)) {
     pp.pair = 1;                                                   // see IgemmParams::pair
     pp.nkb = 2 * p.kh * p.kw * (p.Cin / 64);
   }
-  const int ntn_host = (p.Cout + bn - 1) / bn;
   if (p.h2_w != nullptr) {                     // HEAD2 epilogue: the strict-precision predictor GEMM (see IgemmParams)
-    if (!(a_tma && (bn == 128 || bn == 256) && pp.pair && p.Cout % 256 == 0 && p.h2_part != nullptr && p.Cout / 256 <= 12)) {
-      set_error("igemm2 HEAD2: needs the pair-schedule TMA path with 128/256-column tiles and Cout a multiple of 256");
+    if (!(a_tma && pp.pair && p.Cout % 256 == 0 && p.h2_part != nullptr && p.Cout / 256 <= 12)) {
+      set_error("igemm2 HEAD2: needs the pair-schedule TMA path and Cout a multiple of 256");
       return -1;
     }
-    if (bn == 256) return launch2_cfg<256, MODE_CONV_TMA, 4, 2>(tw, ty, tx, pp, 0, st);
     return launch2_cfg<128, MODE_CONV_TMA, 4, 2>(tw, ty, tx, pp, 0, st);
   }
   if (p.split_out && use_tma_store) {          // staged hi/lo tiles: the SPLIT instantiations (N tiles of 64 / 128 only)
@@ -1119,16 +906,17 @@ int launch_igemm2(const IgemmParams& p, const __half* wp, int n_pad, int k_pad, 
     if (bn == 128) return launch2_cfg<128, MODE_CONV, 4, 1>(tw, ty, tx, pp, use_tma_store, st);
   }
   if (mode == MODE_DCN && p.split_in) { set_error("dcn igemm: strict precision needs the staged TMA-store epilogue"); return -1; }
+  if (mode == MODE_DCN) {                      // 16 gather warps for 64 / 128-column tiles, 8 for Cout <= 32
+    if (bn == 16) return launch2_cfg<16, MODE_DCN, 8>(tw, ty, tx, pp, use_tma_store, st);
+    if (bn == 32) return launch2_cfg<32, MODE_DCN, 8>(tw, ty, tx, pp, use_tma_store, st);
+    if (bn == 64) return launch2_cfg<64, MODE_DCN, 16>(tw, ty, tx, pp, use_tma_store, st);
+    if (bn == 128) return launch2_cfg<128, MODE_DCN, 16>(tw, ty, tx, pp, use_tma_store, st);
+  }
 #define MF_DISPATCH2(BN)                                                                          \
   if (bn == BN) {                                                                                 \
-    if (mode == MODE_DCN) return launch2_cfg<BN, MODE_DCN, 8>(tw, ty, tx, pp, use_tma_store, st);  \
-    if (a_tma && BN == 128 && pp.kc == 64 && pp.nkb <= AS_MAX_KB && ntn_host >= 4 && g_tunable[6] == 1)      \
-      return launch2_cfg<128, MODE_CONV_TMA_AS, 4>(tw, ty, tx, pp, use_tma_store, st);             \
     if (a_tma) return launch2_cfg<BN, MODE_CONV_TMA, 4>(tw, ty, tx, pp, use_tma_store, st);        \
     return launch2_cfg<BN, MODE_CONV, 4>(tw, ty, tx, pp, use_tma_store, st);                       \
   }
-  if (mode == MODE_DCN && g_tunable[7] != 2 && bn == 64) return launch2_cfg<64, MODE_DCN, 16>(tw, ty, tx, pp, use_tma_store, st);
-  if (mode == MODE_DCN && g_tunable[7] != 2 && bn == 128) return launch2_cfg<128, MODE_DCN, 16>(tw, ty, tx, pp, use_tma_store, st);
   MF_DISPATCH2(16)
   MF_DISPATCH2(32)
   MF_DISPATCH2(64)

@@ -21,7 +21,6 @@ struct NormConsts { float mean[3], stdv[3]; int to_bgr; };
 __global__ void __launch_bounds__(256) preprocess_u8_kernel(const unsigned char* const* __restrict__ src,
                                                             const int* __restrict__ hw, const int* __restrict__ flip, int B,
                                                             int H, int W, NormConsts k, float* __restrict__ out) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   const long long HW = static_cast<long long>(H) * W;
   if (i >= B * HW) return;
@@ -57,7 +56,6 @@ int launch_preprocess_u8(const unsigned char* const* src, const int* hw, const i
 // obj: int32 [B][max_objs][6] = (valid, cls, cx, cy, rx, ry); hm: fp32 [B][ncls][H][W]
 __global__ void __launch_bounds__(256) draw_heatmap_kernel(const int* __restrict__ obj, int B, int max_objs, int ncls, int H,
                                                            int W, float* __restrict__ hm) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   const long long plane = static_cast<long long>(H) * W;
   if (i >= B * ncls * plane) return;

@@ -6,7 +6,7 @@
 
 namespace mf {
 
-enum { MODE_CONV = 0, MODE_DCN = 1, MODE_CONV_TMA = 2, MODE_CONV_TMA_AS = 3, MODE_CONV_PATCH = 4 };
+enum { MODE_CONV = 0, MODE_DCN = 1, MODE_CONV_TMA = 2 };
 enum { ACT_NONE = 0, ACT_RELU = 1, ACT_LEAKY = 2, ACT_OFFMASK = 3 };
 enum { OUT_F16_NHWC = 0, OUT_F32_NHWC = 1, OUT_F32_NCHW = 2 };
 
@@ -19,7 +19,6 @@ struct IgemmParams {
   int M;        // B*Ho*Wo
   int K_real;   // kh*kw*Cin
   int nkb;      // ceil(K_real / 64)
-  int kc;       // MODE_CONV_TMA: channels per im2col box (8/16/32/64), 64/kc taps per K block; 0 otherwise
   // DCN: per output pixel 18 offsets (dy,dx per tap) + 9 masks (already sigmoid-ed), fp32, row stride om_ld
   const float* offmask;
   int om_ld;
@@ -40,7 +39,7 @@ struct IgemmParams {
   int split_in, split_out;
   int x_lo, res_lo, y_lo;
   int cw;       // split_in: channels per chunk = min(Cin, 64)
-  // pair schedule (set by launch_igemm2 for split_in with 64-channel K blocks): per (tap, chunk) only TWO stages are filled,
+  // pair schedule (set by launch_igemm2 for split_in on the im2col-TMA and DCN paths): per (tap, chunk) only TWO stages are filled,
   // (A_hi, W_hi) and (A_lo, W_lo), and the MMA warp issues the three products A_hi W_hi, A_lo W_hi, A_hi W_lo across them -
   // one third less operand traffic into shared memory than the K-concatenation (which loads A_hi and W_hi twice).
   // nkb then counts stage fills = 2 * taps * Cin / 64.

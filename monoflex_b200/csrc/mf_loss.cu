@@ -272,7 +272,6 @@ __device__ void block_sum(float (&v)[N], float* sm /* [32*N] */) {
 __global__ void __launch_bounds__(256) loss_forward_kernel(const float* __restrict__ reg, const float* __restrict__ obj,
                                                            const float* __restrict__ img, const float* __restrict__ focal2,
                                                            LossCfg c, float* __restrict__ out, float* __restrict__ ws) {
-  pdl_wait();
   __shared__ float sm[32 * (NTERM + NLOG)];
   __shared__ float s_coef[NTERM];
   __shared__ float s_fukp[64];
@@ -364,7 +363,6 @@ __global__ void __launch_bounds__(128) loss_backward_kernel(const float* __restr
                                                             const float* __restrict__ img, const float* __restrict__ ws,
                                                             const float* __restrict__ gw, LossCfg c,
                                                             float* __restrict__ grad_reg) {
-  pdl_wait();
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const int slots = c.B * c.M;
   if (t >= slots * 50) return;

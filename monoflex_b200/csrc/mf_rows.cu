@@ -50,7 +50,6 @@ template <int BLOCK_N>
 __global__ void __launch_bounds__(192, 2)
 rows_conv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_w,
                  const __grid_constant__ RowsParams p) {
-  pdl_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int stage_bytes = p.nseg * SEG_BYTES;                 // multiple of 128
@@ -84,7 +83,6 @@ rows_conv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_consta
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();
 
   if (warp == 0) {
     // ================================================================ TMA: resident weights, then row segments per tile

@@ -73,7 +73,6 @@ int launch_pack_conv_weight_split(const float* w, int Cout, int Cin, int kh, int
 // channels [hi(3) | lo(3) | hi(3) | 0 x 7]: the 7x7 stem then is an ORDINARY 16-channel convolution whose per-tap weights are
 // [W_hi | W_hi | W_lo | 0] (engine.py), i.e. the three split products in one pass over 16 instead of 3 x 8 channels.
 __global__ void pack_image_split_kernel(const float* __restrict__ x, __half* __restrict__ y, int B, int C, long long HW) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B * HW) return;
   const long long b = i / HW, pix = i - b * HW;
@@ -104,7 +103,6 @@ int launch_pack_image_split(const float* x, __half* y, int B, int C, int H, int 
 
 // image -> ONE 16-byte-pixel plane [hi3 | lo3 | 0 0] for the row-segment stem kernel (mf_rows.cu, in_mode 1)
 __global__ void pack_image_pair8_kernel(const float* __restrict__ x, __half* __restrict__ y, int B, int C, long long HW) {
-  pdl_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B * HW) return;
   const long long b = i / HW, pix = i - b * HW;
@@ -133,7 +131,6 @@ int launch_pack_image_pair8(const float* x, __half* y, int B, int C, int H, int 
 // ---------------------------------------------------------------- MaxPool2d(2) on hi/lo rows
 __global__ void maxpool2_split_kernel(const __half* __restrict__ x, int x_lo, __half* __restrict__ y, int y_lo, int B, int H,
                                       int W, int C, int x_ld, int y_ld) {
-  pdl_wait();
   const int Ho = H / 2, Wo = W / 2, CV = C / 8;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Ho * Wo * CV) return;
@@ -166,7 +163,6 @@ int launch_maxpool2_split(const __half* x, int x_lo, __half* y, int y_lo, int B,
 __global__ void upsample_add_split_kernel(const __half* __restrict__ x, int x_lo, const float* __restrict__ w,
                                           const __half* __restrict__ skip, int skip_lo, __half* __restrict__ y, int y_lo, int B,
                                           int Hi, int Wi, int C, int f, int x_ld, int skip_ld, int y_ld) {
-  pdl_wait();
   const int Ho = Hi * f, Wo = Wi * f, CV = C / 8, k = 2 * f, pad = f / 2;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * Ho * Wo * CV) return;
@@ -251,7 +247,6 @@ int launch_upsample_add_split(const __half* x, int x_lo, const float* w, const _
 __global__ void edge_gather_split_kernel(const __half* __restrict__ feat, int feat_ld, int feat_lo, int ch_a, int ch_b,
                                          const long long* __restrict__ edge_idx, __half* __restrict__ ea,
                                          __half* __restrict__ eb, int B, int H, int W, int K, int out_w, int out_h) {
-  pdl_wait();
   const int CV = 32;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * (K + 2) * CV * 2) return;
@@ -304,7 +299,6 @@ __global__ void edge_head_add_split_kernel(const __half* __restrict__ t, int t_l
                                            const float* __restrict__ bias, int n_out, const long long* __restrict__ edge_idx,
                                            const long long* __restrict__ edge_len, float* __restrict__ out, int out_ctot,
                                            int out_ch0, int B, int K, int H, int W) {
-  pdl_wait();
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (warp >= B * K) return;
   const int b = warp / K, e = warp - b * K;
@@ -332,7 +326,6 @@ int launch_edge_head_add_split(const __half* t, int t_ld, int t_lo, const float*
 
 // hi/lo rows -> fp32 NCHW (tests / feature-map export): y = float(hi) + float(lo)
 __global__ void split_to_nchw_kernel(const __half* __restrict__ x, int x_ld, int x_lo, float* __restrict__ y, int C, int HW) {
-  pdl_wait();
   __shared__ float tile[32][33];
   const int b = blockIdx.z, p0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
   for (int i = threadIdx.y; i < 32; i += blockDim.y) {

@@ -45,7 +45,6 @@ __global__ void __launch_bounds__(256) adamw_arena_kernel(float* __restrict__ p,
                                                           float* __restrict__ m, float* __restrict__ v,
                                                           const float* __restrict__ chunk_lr, long long n_chunks,
                                                           AdamwConsts k) {
-  pdl_wait();
   constexpr int VEC_PER_CHUNK = MF_ADAMW_CHUNK / 4;
   const long long n_vec = n_chunks * VEC_PER_CHUNK;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_vec;
@@ -190,7 +189,6 @@ int launch_adamw_arena(float* p, const float* g, float* m, float* v, const float
 struct AdamwDyn { float bc1, rsqrt_bc2; int skip, pad; };
 
 __global__ void __launch_bounds__(256) grad_finite_kernel(const float* __restrict__ g, long long n_vec, long long* state) {
-  pdl_wait();
   bool bad = false;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_vec;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -202,7 +200,6 @@ __global__ void __launch_bounds__(256) grad_finite_kernel(const float* __restric
   if (__syncthreads_or(bad ? 1 : 0) && threadIdx.x == 0) atomicExch(reinterpret_cast<unsigned long long*>(state + 1), 1ull);
 }
 __global__ void adamw_prepare_kernel(long long* state, AdamwDyn* dyn, float beta1, float beta2, int check) {
-  pdl_wait();
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   const bool skip = check != 0 && state[1] != 0;
   if (skip) state[2] += 1; else state[0] += 1;
@@ -218,7 +215,6 @@ __global__ void __launch_bounds__(256) adamw_arena_dyn_kernel(float* __restrict_
                                                               float* __restrict__ m, float* __restrict__ v,
                                                               const float* __restrict__ chunk_lr, long long n_chunks,
                                                               AdamwConsts k, const AdamwDyn* __restrict__ dyn) {
-  pdl_wait();
   if (dyn->skip) return;
   k.bc1 = dyn->bc1;
   k.rsqrt_bc2 = dyn->rsqrt_bc2;
@@ -263,7 +259,6 @@ int launch_adamw_arena_dyn(float* p, const float* g, float* m, float* v, const f
 //       = -(1-t)^4 ( 2 p log(1-p) - p^2 / (1-p) )                   at 0 <= t < 1,   0 elsewhere (ignored pixels, t = -1)
 __global__ void focal_loss_backward_kernel(const float* __restrict__ pred, const float* __restrict__ tgt, long long n,
                                            const float* __restrict__ scale, float* __restrict__ grad) {
-  pdl_wait();
   const float s = __ldg(scale);
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {

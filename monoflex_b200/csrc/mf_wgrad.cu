@@ -237,8 +237,8 @@ int launch_conv_wgrad(const __half* x, int x_ld, int B, int H, int W, int Cin, c
               Cout, kh, kw, stride);
     return -1;
   }
-  if (Cin == 16 && Cout == 16 && stride == 1 && kh == kw && (kh == 3 || kh == 7) && pad_h == kh / 2 && pad_w == kh / 2 &&
-      g_tunable[10] == 0)                                   // full-resolution stem layers: all reduction, no tile (mf_wgrad_narrow.cu)
+  // full-resolution stem layers: all reduction, no tile (mf_wgrad_narrow.cu)
+  if (Cin == 16 && Cout == 16 && stride == 1 && kh == kw && (kh == 3 || kh == 7) && pad_h == kh / 2 && pad_w == kh / 2)
     return launch_conv_wgrad_narrow(x, x_ld, B, H, W, dy, dy_ld, kh, dw, st);
   const int aw = Cin < 64 ? Cin : 64, bw = Cout < 64 ? Cout : 64;
   WgradParams p;

@@ -127,9 +127,8 @@ class DLA(nn.Module):
 
     def plan(self, P, x8):
         """DLA.forward (:324-331). x8: image already packed to NHWC fp16 with 8 channels (3 real + 5 zero)."""
-        import os
         rows_ok = (len(self.level0) == 3 and len(self.level1) == 3 and self.channels[0] == 16 and x8.W % 2 == 0 and
-                   self.level1[0].stride[0] == 2 and os.environ.get("MF_NO_ROWS_STEM", "0") != "1" and not P.train)
+                   self.level1[0].stride[0] == 2 and not P.train)
         y = []
         if P.strict and rows_ok:
             # strict precision on the row-segment kernel: x8 is the image pair plane [hi3 | lo3 | 0 0] (mf_pack_image_pair8);
@@ -263,8 +262,7 @@ class DLASeg(nn.Module):
     def build_plan(self, B, H, W, device):
         strict = (not self.training) and self._precision() == "strict"
         P = engine.Plan(device, train=self.training, strict=strict)
-        import os
-        self._strict_rows = strict and os.environ.get("MF_NO_ROWS_STEM", "0") != "1" and W % 2 == 0
+        self._strict_rows = strict and W % 2 == 0
         x8 = P.act(B, H, W, 8 if (self._strict_rows or not strict) else 16, split=False)
         P.image_pack = "mf_pack_image_pair8" if self._strict_rows else ("mf_pack_image_split" if strict else "mf_pack_image")
         levels = self.base.plan(P, x8)

@@ -103,12 +103,11 @@ class _predictor(nn.Module):
         if self.enable_edge_fusion:
             off_ch0 = ch0s[self.offset_index[0]] + sum(h.weight.shape[0] for h in
                                                        list(self.reg_heads[self.offset_index[0]])[:self.offset_index[1]])
-        import os
         # strict precision runs the generic split GEMMs: the nine 3x3 convs as one N = 2304 layer whose hi/lo hidden map goes
         # through HBM once (2.3 GB at B = 8), then the 1x1 heads on its channel slices
-        fused = not P.train and not strict and os.environ.get("MF_NO_FUSED_HEAD", "0") != "1" and hc == 256 and feat.C % 64 == 0 and \
+        fused = not P.train and not strict and hc == 256 and feat.C % 64 == 0 and \
             all(sum(h.weight.shape[0] for h in heads) <= 32 for heads in self.reg_heads) and self.num_classes <= 32
-        head2 = not P.train and strict and os.environ.get("MF_NO_HEAD2", "0") != "1" and hc == 256 and feat.C % 64 == 0 and \
+        head2 = not P.train and strict and hc == 256 and feat.C % 64 == 0 and \
             (H * W) % 4 == 0 and len(branches) <= 12 and self.num_classes <= 32 and \
             all(sum(h.weight.shape[0] for h in heads) <= 32 for heads in self.reg_heads)
         if head2:
@@ -188,7 +187,7 @@ class _predictor(nn.Module):
             arr_ct, arr_nc, arr_hc = (ctypes.c_int * nb)(*out_ctot), (ctypes.c_int * nb)(*out_nch), (ctypes.c_int * nb)(*hid_col)
             P.edge_idx = torch.zeros(B, K_edge, 2, dtype=torch.long, device=dev)
             hid_mask = None
-            if self.enable_edge_fusion and os.environ.get("MF_HID_FULL_STORE", "0") != "1":
+            if self.enable_edge_fusion:
                 # only the border pixels the edge fusion gathers need their hidden activations in HBM
                 hid_mask = torch.zeros(B * H * W, dtype=torch.uint8, device=dev)
                 ow_, oh_ = self.output_width, self.output_height

@@ -16,7 +16,7 @@ from oracle import monoflex_oracle as mo
 
 pytestmark = pytest.mark.gpu
 
-DCN_CASES_EARLY = [(1, 64, 12, 20, 64), (2, 128, 7, 9, 64), (1, 256, 6, 10, 128), (1, 512, 4, 6, 256), (2, 64, 24, 40, 64), (2, 64, 24, 48, 64), (1, 128, 16, 32, 64)]  # last two: offset conv in patch mode (strict)
+DCN_CASES_EARLY = [(1, 64, 12, 20, 64), (2, 128, 7, 9, 64), (1, 256, 6, 10, 128), (1, 512, 4, 6, 256), (2, 64, 24, 40, 64), (2, 64, 24, 48, 64), (1, 128, 16, 32, 64)]  # last two: maps that tile exactly into 16 x 8 pixel blocks
 CONV_CASES = [
     # B, Cin, H, W, Cout, k, stride, pad, act, residual
     (2, 16, 12, 20, 16, 3, 1, 1, engine.ACT_RELU, False),      # level0-like, N tile 16
@@ -30,16 +30,16 @@ CONV_CASES = [
     (3, 64, 7, 11, 64, 3, 1, 1, engine.ACT_RELU, True),        # tiles wrap across rows and images (im2col traversal)
     (2, 64, 17, 23, 128, 3, 2, 1, engine.ACT_RELU, False),     # stride 2 on odd sizes
     (2, 128, 5, 300, 64, 3, 1, 1, engine.ACT_NONE, False),     # wide rows: several 128-pixel tiles per image row
-    (2, 32, 12, 20, 64, 3, 2, 1, engine.ACT_RELU, False),      # Cin 32: 64-byte im2col boxes, 2 taps per K block
-    (1, 16, 33, 47, 32, 3, 1, 1, engine.ACT_RELU, True),       # Cin 16: 32-byte boxes, 4 taps per K block, ragged
-    (2, 64, 19, 23, 640, 3, 1, 1, engine.ACT_LEAKY, False),    # head-like: A-stationary mode (5 N tiles, 9 K blocks, 7 m-tiles)
-    (1, 64, 40, 500, 512, 1, 1, 0, engine.ACT_RELU, False),    # A-stationary with a single resident K block, many m-tiles
-    # strict precision: maps that tile into 16 x 8 patches take the patch mode (kx-shifted A slots, csrc/mf_igemm2.cu)
-    (2, 64, 16, 32, 64, 3, 1, 1, engine.ACT_RELU, True),       # patch mode, N tile 64, residual, image borders in every tile
-    (1, 128, 24, 48, 128, 3, 1, 1, engine.ACT_RELU, False),    # patch mode, two 64-channel chunks, N tile 128 (4-slot ring)
-    (1, 64, 16, 32, 256, 3, 1, 1, engine.ACT_LEAKY, False),    # patch mode, two N tiles, slots re-loaded per N tile
-    (1, 128, 8, 32, 64, 3, 1, 1, engine.ACT_NONE, True),       # patch mode, 128 -> 64
-    (2, 64, 96, 160, 64, 3, 1, 1, engine.ACT_RELU, True),      # patch mode, 240 m-tiles: every CTA wraps its slot / stage rings
+    (2, 32, 12, 20, 64, 3, 2, 1, engine.ACT_RELU, False),      # Cin 32: cp.async gather, 2 taps per K block
+    (1, 16, 33, 47, 32, 3, 1, 1, engine.ACT_RELU, True),       # Cin 16: cp.async gather, 4 taps per K block, ragged
+    (2, 64, 19, 23, 640, 3, 1, 1, engine.ACT_LEAKY, False),    # head-like: 5 N tiles, 9 K blocks, 7 m-tiles
+    (1, 64, 40, 500, 512, 1, 1, 0, engine.ACT_RELU, False),    # a single K block, many m-tiles
+    # maps that tile exactly into 16 x 8 pixel blocks
+    (2, 64, 16, 32, 64, 3, 1, 1, engine.ACT_RELU, True),       # N tile 64, residual, image borders in every tile
+    (1, 128, 24, 48, 128, 3, 1, 1, engine.ACT_RELU, False),    # two 64-channel chunks, N tile 128
+    (1, 64, 16, 32, 256, 3, 1, 1, engine.ACT_LEAKY, False),    # two N tiles
+    (1, 128, 8, 32, 64, 3, 1, 1, engine.ACT_NONE, True),       # 128 -> 64
+    (2, 64, 96, 160, 64, 3, 1, 1, engine.ACT_RELU, True),      # 240 m-tiles: every CTA wraps its stage ring
 ]
 
 
@@ -118,23 +118,6 @@ def run_conv_strict(case, seed=0):
 @pytest.mark.parametrize("case", STRICT_CONV_CASES)
 def test_conv_strict_pairs(case):
     y, ref = run_conv_strict(case)
-    assert rel_err(y, ref) < STRICT_TOL
-
-
-PATCH_CASES = [c for c in STRICT_CONV_CASES if c[1] % 64 == 0 and c[5] == 3 and c[6] == 1 and c[2] % 8 == 0 and c[3] % 16 == 0]
-
-
-@pytest.mark.parametrize("case", PATCH_CASES)
-def test_conv_strict_patch_mode(case):
-    """the opt-in patch mode of the pair GEMM (kx-shifted A slots instead of nine im2col boxes, tunable 13 / MF_PATCH)"""
-    from monoflex_b200 import _lib
-    assert len(PATCH_CASES) >= 5
-    lib = _lib.load()
-    assert lib.mf_set_tunable(13, 1) == 0
-    try:
-        y, ref = run_conv_strict(case)
-    finally:
-        lib.mf_set_tunable(13, 0)
     assert rel_err(y, ref) < STRICT_TOL
 
 
